@@ -15,6 +15,9 @@ samples (synthetic data: the latents ARE the data).
   parity    size-independent properties of the timed result + a small-N run of the same config compared with the oracle
   cpu_baseline  the reference arm on a bounded sample, run as a subprocess (CPU only) after the timed region
 
+--dump-outputs DIR writes the arrays of the last timed step as DIR/<name>.npy; the inputs are seeded, so two builds run with the
+same arguments can be compared output for output.
+
 --impl reference times the UNMODIFIED reference (baseline/_ref = the *.py tree of harskish/ganspace, installed by
 __graft_entry__.build(); oracle/ref_harness.py) through its own decomposition.get_or_compute on the host cores, one bounded
 sample of the workload per step (default N=100_000 of the 1e6: the path's cost is linear in the number of 10k batches).  The
@@ -267,6 +270,24 @@ def _props(out):
             "finite": bool(all(np.isfinite(v).all() for v in out.values()))}
 
 
+DUMP_BYTES = 64 << 20
+
+
+def _dump_outputs(arrays, out_dir):
+    """--dump-outputs: the float32 arrays compute_arrays() returned, as <out_dir>/<name>.npy, so that two builds can be compared
+    output for output.  Each array gets an equal share of DUMP_BYTES; a larger one (act_comp of a conv layer: 168 MB at convs.4)
+    is replaced by a sample of its flattened elements at positions drawn from a fixed seed, the same positions on every run."""
+    import numpy as np
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    share = DUMP_BYTES // len(arrays)
+    for name, a in arrays.items():
+        if a.nbytes > share:
+            idx = np.random.default_rng(0).choice(a.size, share // a.itemsize, replace=False)
+            a = a.reshape(-1)[np.sort(idx)]
+        np.save(out_dir / f"{name}.npy", a)
+
+
 def run_ours(args):
     import numpy as np
     import torch
@@ -340,7 +361,7 @@ def run_ours(args):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        quiet(lambda: decomposition.compute_arrays(cfg(), inst))
+        last = quiet(lambda: decomposition.compute_arrays(cfg(), inst))
     e1.record()
     barrier()
     dev_ms = e0.elapsed_time(e1) / args.steps
@@ -362,6 +383,8 @@ def run_ours(args):
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     dev_ms, e2e_ms = float(t[0]), float(t[1])
+    if args.dump_outputs and rank == 0:
+        _dump_outputs(last, args.dump_outputs)
 
     # ---- the roofline kernel alone (outside the timed region): same rows, nothing else on the GPU -------------------------
     isolated = None
@@ -479,7 +502,14 @@ def main():
     ap.add_argument("--no-ref-full", dest="ref_full", action="store_false")
     ap.add_argument("--no-cpu-baseline", dest="no_cpu_baseline", action="store_true")
     ap.add_argument("--no-parity", dest="no_parity", action="store_true")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the arrays of the last step as DIR/<name>.npy (float32, at most 64 MB "
+                         "in all; a larger array is replaced by a fixed, seeded sample of its elements)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.impl == "reference":
         os.environ["CUDA_VISIBLE_DEVICES"] = ""          # the reference picks 'cuda' when it sees one (decomposition.py:163-164)
         run_reference(args)

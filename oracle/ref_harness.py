@@ -28,10 +28,18 @@ REF_SRC = Path(os.environ.get("GANSPACE_REFERENCE", "/root/reference"))
 REF_DST = REPO / "baseline" / "_ref"
 
 
+def _is_file(p: Path) -> bool:
+    """Path.is_file() that answers False, rather than raising, for a path the user may not read."""
+    try:
+        return p.is_file() and os.access(p, os.R_OK)
+    except OSError:
+        return False
+
+
 def install_ref(src: Path = REF_SRC, dst: Path = REF_DST) -> bool:
-    """Mirror the reference's *.py tree into baseline/_ref (idempotent).  False when the source is absent."""
+    """Mirror the reference's *.py tree into baseline/_ref (idempotent).  False when the source is absent or unreadable."""
     src = Path(src)
-    if not (src / "decomposition.py").is_file():
+    if not _is_file(src / "decomposition.py"):
         return False
     n = 0
     for p in src.rglob("*.py"):
@@ -50,7 +58,7 @@ def install_ref(src: Path = REF_SRC, dst: Path = REF_DST) -> bool:
 def ref_dir():
     """Directory of an importable reference tree: /root/reference here, baseline/_ref on the GPU box; None if neither."""
     for d in (REF_SRC, REF_DST):
-        if (d / "decomposition.py").is_file() and (d / "models" / "wrappers.py").is_file():
+        if _is_file(d / "decomposition.py") and _is_file(d / "models" / "wrappers.py"):
             return d
     return None
 
