@@ -36,6 +36,12 @@ SIGNATURES = {
     "gsb_mapping_status": (_I, [_P, _I, _I, _P]),
     "gsb_linear_forward": (_I, [_P, _P, _P, _P, _L, _I, _I, _I, _P, _Z, _P]),
     "gsb_linear_workspace_bytes": (_Z, [_L, _I, _I, _I]),
+    "gsb_leaky_relu": (_I, [_P, _P, _L, _F, _P]),
+    "gsb_sg1_packed_bytes": (_Z, [_P, _I, _I]),
+    "gsb_sg1_pack": (_I, [_P, _I, _I, _P, _P, _P, _Z, _P]),
+    "gsb_sg1_workspace_bytes": (_Z, [_P, _I, _I, _I, _L]),
+    "gsb_sg1_forward": (_I, [_P, _P, _I, _I, _I, _I, _P, _I, _L, _P, _L, _P, _Z, _P]),
+    "gsb_sg1_status": (_I, [_P, _P, _I, _I, _P]),
     "gsb_batch_stats_workspace_bytes": (_Z, [_L, _I]),
     "gsb_batch_stats": (_I, [_P, _L, _I, _L, _P, _P, _P, _Z, _P]),
     "gsb_batch_stats_multi_workspace_bytes": (_Z, [_I, _L, _I]),
@@ -94,6 +100,13 @@ class ToRGBDesc(C.Structure):
     """``gsb_to_rgb`` of include/ganspace_b200.h."""
     _fields_ = [("conv_weight", C.c_void_p), ("mod_weight", C.c_void_p), ("mod_bias", C.c_void_p), ("bias", C.c_void_p),
                 ("cin", C.c_int)]
+
+
+class SG1LayerDesc(C.Structure):
+    """``gsb_sg1_layer`` of include/ganspace_b200.h."""
+    _fields_ = [("kind", C.c_int), ("cin", C.c_int), ("cout", C.c_int), ("res_out", C.c_int), ("weight", C.c_void_p),
+                ("bias", C.c_void_p), ("noise_weight", C.c_void_p), ("noise", C.c_void_p), ("style_weight", C.c_void_p),
+                ("style_bias", C.c_void_p)]
 
 
 class NativeError(RuntimeError):
@@ -425,6 +438,18 @@ def linear(x: torch.Tensor, w: torch.Tensor, bias: torch.Tensor = None, lrelu: b
     return y.reshape(*x.shape[:-1], N)
 
 
+def leaky_relu(x: torch.Tensor, slope: float = 0.2) -> torch.Tensor:
+    """leaky_relu(x, slope) without gain (StyleGAN's G_mapping activation)."""
+    lib = load()
+    assert x.is_cuda and x.dtype == torch.float32
+    x2 = x.contiguous()
+    y = torch.empty_like(x2)
+    with torch.cuda.device(x.device):
+        _check(lib.gsb_leaky_relu(_ptr(x2), _ptr(y), x2.numel(), float(slope), _stream()), "gsb_leaky_relu")
+    instrument.count(1)
+    return y.reshape(x.shape)
+
+
 def mapping_pixelnorm(z: torch.Tensor) -> torch.Tensor:
     """PixelNorm alone (stylegan2-pytorch/model.py:14-19)."""
     lib = load()
@@ -726,6 +751,86 @@ class LinregAccumulator:
                                                  _stream()), "gsb_linreg_solve_pinv")
             instrument.count(9)
         return M, zmean
+
+
+class PackedSG1:
+    """StyleGAN (v1) synthesis network packed for csrc/synthesis_sg1.cu (gsb_sg1_pack).
+
+    ``layers``: dicts with kind ('const' | 'same' | 'nearest' | 'fused'), weight (const [c,4,4] or conv weight [co,ci,3,3]),
+    bias [co], noise_weight [co], noise [r,r], style_weight [2co, dlatent], style_bias [2co] (fp32 tensors), cin, cout, res_out;
+    ``rgb_weight`` [3, c_last] and ``rgb_bias`` [3] of torgb."""
+    KINDS = {"const": 0, "same": 1, "nearest": 2, "fused": 3}
+    STOPS = {"epi": 0, "conv": 1, "style": 2, "image": 3}
+
+    def __init__(self, layers, rgb_weight: torch.Tensor, rgb_bias: torch.Tensor, dlatent: int = 512):
+        lib = load()
+        self.device = require_cuda(rgb_weight.device)
+        self.dlatent = int(dlatent)
+        self.n_layers = len(layers)
+        self.desc = (SG1LayerDesc * self.n_layers)()
+        self.shapes = []                        # (res_out, cout) per layer
+        f32 = lambda t: t.detach().to(self.device, torch.float32).contiguous()
+        keep = []
+        for i, L in enumerate(layers):
+            ts = {k: f32(L[k]) for k in ("weight", "bias", "noise_weight", "noise", "style_weight", "style_bias")}
+            keep.append(ts)
+            d = self.desc[i]
+            for k, t in ts.items():
+                setattr(d, k, t.data_ptr())
+            d.kind, d.cin, d.cout, d.res_out = self.KINDS[L["kind"]], int(L["cin"]), int(L["cout"]), int(L["res_out"])
+            assert ts["noise"].numel() == d.res_out ** 2 and ts["style_weight"].shape == (2 * d.cout, self.dlatent)
+            self.shapes.append((d.res_out, d.cout))
+        rw, rb = f32(rgb_weight).reshape(3, -1), f32(rgb_bias).reshape(3)
+        nbytes = lib.gsb_sg1_packed_bytes(self.desc, self.n_layers, self.dlatent)
+        if nbytes == 0:
+            raise NativeError(f"gsb_sg1_packed_bytes: {lib.gsb_last_error().decode()}")
+        self.packed = torch.empty(nbytes, dtype=torch.uint8, device=self.device)
+        with torch.cuda.device(self.device):
+            _check(lib.gsb_sg1_pack(self.desc, self.n_layers, self.dlatent, _ptr(rw), _ptr(rb), _ptr(self.packed),
+                                    self.packed.numel(), _stream()), "gsb_sg1_pack")
+            torch.cuda.current_stream().synchronize()      # the temporaries above may be freed after this returns
+
+    def out_dims(self, n_run: int, stop: str) -> int:
+        r, co = self.shapes[n_run - 1]
+        return {"epi": r * r * co, "conv": r * r * co, "style": 2 * co, "image": 3 * r * r}[stop]
+
+    def forward(self, w_layers: torch.Tensor, n_run: int, stop: str = "epi", out: torch.Tensor = None) -> torch.Tensor:
+        """Result ``stop`` of layer ``n_run - 1`` for per-layer latents w_layers [Lw, n, dlatent] (layer j reads entry
+        min(j, Lw - 1); Lw = 1: one latent for all layers): fp32 rows [n, out_dims] (NHWC for 'epi' / 'conv', NCHW for
+        'image'); ``out`` may be a row-strided 2-D view (e.g. the batch rows of the large-d IPCA buffer)."""
+        lib = load()
+        assert w_layers.is_cuda and w_layers.dtype == torch.float32 and w_layers.dim() == 3 and w_layers.shape[2] == self.dlatent
+        w_layers = w_layers.contiguous()
+        n, d, code = w_layers.shape[1], self.out_dims(n_run, stop), self.STOPS[stop]
+        if out is None:
+            out = torch.empty((n, d), dtype=torch.float32, device=w_layers.device)
+        assert out.is_cuda and out.dtype == torch.float32 and out.shape == (n, d) and out.stride(1) == 1
+        ws_bytes = lib.gsb_sg1_workspace_bytes(self.desc, self.n_layers, n_run, code, n)
+        ws = scratch.get("synthesis_sg1", ws_bytes, w_layers.device)
+        with torch.cuda.device(w_layers.device), instrument.section("synthesis_sg1"):
+            _check(lib.gsb_sg1_forward(_ptr(self.packed), self.desc, self.n_layers, self.dlatent, n_run, code, _ptr(w_layers),
+                                       w_layers.shape[0], n, C.c_void_p(out.data_ptr()), out.stride(0), _ptr(ws), ws.numel(),
+                                       _stream()), "gsb_sg1_forward")
+        # per layer: 1 style launch; per chunk of samples: GEMM + gather (not on the constant layer), epilogue, stats, norm
+        launches = 1 if stop == "style" else n_run + (1 if stop == "image" else 0)
+        if stop != "style":
+            for i in range(n_run):
+                L = self.desc[i]
+                hw_in = (L.res_out // (2 if L.kind >= 2 else 1)) ** 2
+                chunks = -(-n // max(1, 4096 // hw_in))
+                launches += chunks * ((2 if L.kind else 0) + (1 if (stop == "conv" and i == n_run - 1) else 3))
+        instrument.count(launches)
+        instrument.add_rows("synthesis_sg1", n)
+        return out
+
+    def check(self):
+        """Raise if an operand left fp16's range since the pack (synchronises)."""
+        flags = C.c_uint(0)
+        with torch.cuda.device(self.device):
+            _check(load().gsb_sg1_status(_ptr(self.packed), self.desc, self.n_layers, self.dlatent, C.byref(flags)),
+                   "gsb_sg1_status")
+        if flags.value & 1:
+            raise NativeError("StyleGAN synthesis: an activation exceeded fp16 range in the tap-GEMM operands; results are invalid")
 
 
 class PackedSynthesis:

@@ -293,3 +293,21 @@ extern "C" int gsb_linear_forward(const float *d_x, const float *d_w, const floa
     GSB_CHECK_LAUNCH();
     return GSB_OK;
 }
+
+// y = leaky_relu(x, slope), elementwise, without the sqrt(2) gain: StyleGAN's G_mapping activation modules
+// (models/stylegan/model.py:192-193, nn.LeakyReLU(0.2)), run on their own only when a g_mapping child is hooked
+__global__ void leaky_relu_kernel(const float *__restrict__ x, float *__restrict__ y, int64_t n, float slope) {
+    for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+        const float v = x[i];
+        y[i] = v >= 0.f ? v : __fmul_rn(v, slope);
+    }
+}
+
+extern "C" int gsb_leaky_relu(const float *d_x, float *d_y, int64_t n, float slope, gsb_stream_t stream) {
+    GSB_CHECK_ARG(d_x && d_y && n >= 0, "leaky_relu: null pointer or negative n");
+    if (n == 0) return GSB_OK;
+    const int64_t blocks = (n + 255) / 256;
+    leaky_relu_kernel<<<(unsigned)(blocks < 4096 ? blocks : 4096), 256, 0, (cudaStream_t)stream>>>(d_x, d_y, n, slope);
+    GSB_CHECK_LAUNCH();
+    return GSB_OK;
+}

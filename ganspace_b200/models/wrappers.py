@@ -28,7 +28,7 @@ import torch
 from .. import _native
 from ..config import Config
 from ..netdissect.nethook import InstrumentedModel
-from . import stylegan2
+from . import stylegan, stylegan2
 
 INT32_MAX = int(np.iinfo(np.int32).max)
 
@@ -36,6 +36,21 @@ INT32_MAX = int(np.iinfo(np.int32).max)
 def _global_seed() -> int:
     """``np.random.randint(np.iinfo(np.int32).max)`` on NumPy's global legacy state (wrappers.py:169)."""
     return int(np.random.randint(INT32_MAX))
+
+
+def _checkpoint_or_seed(family, rel_path, random_init):
+    """(checkpoint path, random-init seed or None).  The seed is ``random_init``, else env GANSPACE_B200_RANDOM_INIT; without
+    one the checkpoint under $GANCONTROL_CHECKPOINT_DIR must exist (there is no download)."""
+    root = os.environ.get("GANCONTROL_CHECKPOINT_DIR", Path(__file__).parent / "checkpoints")
+    checkpoint = Path(root) / rel_path
+    seed = random_init
+    if seed is None and os.environ.get("GANSPACE_B200_RANDOM_INIT"):
+        seed = int(os.environ["GANSPACE_B200_RANDOM_INIT"])
+    if seed is None and not checkpoint.is_file():
+        raise RuntimeError(
+            f"{family} checkpoint {checkpoint} not found and no network access to download it; pass "
+            "random_init=<seed> (or set GANSPACE_B200_RANDOM_INIT) for random-init weights")
+    return checkpoint, seed
 
 
 class BaseModel(AbstractBaseClass, torch.nn.Module):
@@ -92,24 +107,14 @@ class BaseModel(AbstractBaseClass, torch.nn.Module):
         return self.model.named_modules(*args, **kwargs)
 
 
-class StyleGAN2(BaseModel):
-    CONFIGS = {"ffhq": 1024, "car": 512, "cat": 256, "church": 256, "horse": 256,
-               "bedrooms": 256, "kitchen": 256, "places": 256}
+class _MappedLatentModel(BaseModel):
+    """What StyleGAN and StyleGAN2 share (wrappers.py:167-179, :302-309, :347-366): Z drawn from the NumPy-legacy stream on the
+    device, W = the mapping network (``_mapping_net()``, a module with ``packed()``) applied to it, and the producer
+    interface the decomposition driver uses (``sample_latents_multi``, ``draw_z_async``, ``z_to_latent``,
+    ``check_numerics``)."""
 
-    def __init__(self, device, class_name, truncation=1.0, use_w=False, random_init=None):
-        super().__init__("StyleGAN2", class_name or "ffhq")
-        self.device = _native.require_cuda(device)
-        self.truncation = truncation
-        self.latent_avg = None
-        self.w_primary = use_w
-        assert self.outclass in self.CONFIGS, \
-            f'Invalid StyleGAN2 class {self.outclass}, should be one of [{", ".join(self.CONFIGS.keys())}]'
-        self.resolution = self.CONFIGS[self.outclass]
-        self.name = f"StyleGAN2-{self.outclass}"
-        self.has_latent_residual = True
-        self._random_init = random_init
-        self.load_model()
-        self.set_noise_seed(0)
+    def _mapping_net(self):
+        raise NotImplementedError
 
     def latent_space_name(self):
         return "W" if self.w_primary else "Z"
@@ -120,28 +125,9 @@ class StyleGAN2(BaseModel):
     def use_z(self):
         self.w_primary = False
 
-    def load_model(self):
-        root = os.environ.get("GANCONTROL_CHECKPOINT_DIR", Path(__file__).parent / "checkpoints")
-        checkpoint = Path(root) / f"stylegan2/stylegan2_{self.outclass}_{self.resolution}.pt"
-        seed = self._random_init
-        if seed is None and os.environ.get("GANSPACE_B200_RANDOM_INIT"):
-            seed = int(os.environ["GANSPACE_B200_RANDOM_INIT"])
-        if checkpoint.is_file() and seed is None:
-            self.model = stylegan2.Generator(self.resolution, 512, 8)
-            ckpt = torch.load(checkpoint, map_location="cpu")
-            self.model.load_state_dict(ckpt["g_ema"], strict=False)
-            self.model = self.model.to(self.device)
-            self.latent_avg = ckpt["latent_avg"].to(self.device)
-        elif seed is not None:
-            # the reference's default init, bit-for-bit: parameters are created on the host in the
-            # reference's order under one manual seed, then moved to the device
-            torch.manual_seed(int(seed))
-            self.model = stylegan2.Generator(self.resolution, 512, 8).to(self.device)
-            self.latent_avg = torch.zeros(512, device=self.device)
-        else:
-            raise RuntimeError(
-                f"StyleGAN2 checkpoint {checkpoint} not found and no network access to download it; pass "
-                "random_init=<seed> (or set GANSPACE_B200_RANDOM_INIT) for random-init weights")
+    def set_output_class(self, new_class):
+        if self.outclass != new_class:
+            raise RuntimeError(f"{self.model_name}: cannot change output class without reloading")
 
     def get_latent_shape(self):
         """The reference samples one latent for its shape (wrappers.py:60-61).  The draw from the global NumPy stream that this
@@ -154,7 +140,7 @@ class StyleGAN2(BaseModel):
             seed = _global_seed()
         z = _native.legacy_normal([seed], 512 * n_samples, self.device).view(n_samples, 512)
         if self.w_primary:
-            z = self.model.style(z)
+            z = self._mapping_net()(z)
         return z
 
     def draw_z_async(self, n_samples, seed):
@@ -178,7 +164,7 @@ class StyleGAN2(BaseModel):
 
     def z_to_latent(self, z):
         """What sample_latent does after drawing z (wrappers.py:176-179): the mapping network in W mode."""
-        return self.model.style(z) if self.w_primary else z
+        return self._mapping_net()(z) if self.w_primary else z
 
     def sample_latents_multi(self, n_samples, seeds, out=None, lazy=False):
         """Several ``sample_latent(n_samples, seed=s)`` calls in ONE launch (one CTA per seed);
@@ -194,7 +180,7 @@ class StyleGAN2(BaseModel):
             z = z.view(S * n_samples, 512)
             if not self.w_primary:
                 return z
-            return self.model.style(z) if out is None else self.model.style.packed().forward(z, out=z)
+            return self._mapping_net()(z) if out is None else self._mapping_net().packed().forward(z, out=z)
         # lazy: the streams are generated in launch groups on a side stream (a small first group, so that the first
         # partial_fit group exists after ~1.5 ms instead of after the whole run's RNG); ensure(row_end) waits for the groups
         # that cover rows [0, row_end) and, in W mode, maps them group by group in place.
@@ -243,7 +229,7 @@ class StyleGAN2(BaseModel):
             for side in sides:
                 z.record_stream(side)
                 seeds_dev.record_stream(side)          # read by launches that run long after this function has returned
-        packed = self.model.style.packed() if self.w_primary else None
+        packed = self._mapping_net().packed() if self.w_primary else None
         state = {"g": 0, "keep": seeds_dev}
         free_sms = int(os.environ.get("GANSPACE_B200_LAZY_FREE_SMS", 72 if parts > 1 else 48))
 
@@ -260,16 +246,51 @@ class StyleGAN2(BaseModel):
 
     def check_numerics(self):
         """Raise if a kernel flagged an out-of-range activation since the weights were packed (synchronises)."""
-        self.model.style.packed().check()
+        self._mapping_net().packed().check()
         if getattr(self, "_synth_cache", None) is not None:
             self._synth_cache[1].check()
 
+
+class StyleGAN2(_MappedLatentModel):
+    CONFIGS = {"ffhq": 1024, "car": 512, "cat": 256, "church": 256, "horse": 256,
+               "bedrooms": 256, "kitchen": 256, "places": 256}
+
+    def __init__(self, device, class_name, truncation=1.0, use_w=False, random_init=None):
+        super().__init__("StyleGAN2", class_name or "ffhq")
+        self.device = _native.require_cuda(device)
+        self.truncation = truncation
+        self.latent_avg = None
+        self.w_primary = use_w
+        assert self.outclass in self.CONFIGS, \
+            f'Invalid StyleGAN2 class {self.outclass}, should be one of [{", ".join(self.CONFIGS.keys())}]'
+        self.resolution = self.CONFIGS[self.outclass]
+        self.name = f"StyleGAN2-{self.outclass}"
+        self.has_latent_residual = True
+        self._random_init = random_init
+        self.load_model()
+        self.set_noise_seed(0)
+
+    def _mapping_net(self):
+        return self.model.style
+
+    def load_model(self):
+        checkpoint, seed = _checkpoint_or_seed("StyleGAN2", f"stylegan2/stylegan2_{self.outclass}_{self.resolution}.pt",
+                                               self._random_init)
+        if seed is None:
+            self.model = stylegan2.Generator(self.resolution, 512, 8)
+            ckpt = torch.load(checkpoint, map_location="cpu")
+            self.model.load_state_dict(ckpt["g_ema"], strict=False)
+            self.model = self.model.to(self.device)
+            self.latent_avg = ckpt["latent_avg"].to(self.device)
+        else:
+            # the reference's default init, bit-for-bit: parameters are created on the host in the
+            # reference's order under one manual seed, then moved to the device
+            torch.manual_seed(int(seed))
+            self.model = stylegan2.Generator(self.resolution, 512, 8).to(self.device)
+            self.latent_avg = torch.zeros(512, device=self.device)
+
     def get_max_latents(self):
         return self.model.n_latent
-
-    def set_output_class(self, new_class):
-        if self.outclass != new_class:
-            raise RuntimeError("StyleGAN2: cannot change output class without reloading")
 
     def forward(self, x):
         """wrappers.py:188-192: images in [0, 1] (before clamping) from one latent, a pair, or one latent per layer.  Hooked
@@ -396,6 +417,199 @@ class StyleGAN2(BaseModel):
                 self.noise.append(torch.randn(1, 1, 2 ** i, 2 ** i).to(self.device))
 
 
+class StyleGAN(_MappedLatentModel):
+    """wrappers.py:269-436 (StyleGAN 1, ``models/stylegan/model.py``).  The mapping network ``g_mapping`` runs on the packed
+    mapping kernels and the synthesis network as one fused C-ABI call (models/stylegan.py, csrc/synthesis_sg1.cu).  Hooks on
+    g_mapping retain and edit (the wrapper calls the module, so what its hooks return is what synthesis consumes).  Hooks on
+    the synthesis stop points (blocks, epi1 / epi2, style_mod, style_mod.lin, conv / conv0_up / conv1, torgb, g_synthesis)
+    receive their activations; an edit there would have to be re-fed into the fused chain, which is not built, and raises.  A
+    hook on any other synthesis module (noise, activation, instance_norm, upscale, blur) raises NotImplementedError."""
+    CONFIGS = {"ffhq": 1024, "celebahq": 1024, "bedrooms": 256, "cars": 512, "cats": 256, "vases": 1024, "wikiart": 512,
+               "fireworks": 512, "abstract": 512, "anime": 512, "ukiyo-e": 512}
+
+    def __init__(self, device, class_name, truncation=1.0, use_w=False, random_init=None):
+        super().__init__("StyleGAN", class_name or "ffhq")
+        self.device = _native.require_cuda(device)
+        self.w_primary = use_w
+        assert self.outclass in self.CONFIGS, \
+            f'Invalid StyleGAN class {self.outclass}, should be one of [{", ".join(self.CONFIGS.keys())}]'
+        self.resolution = self.CONFIGS[self.outclass]
+        self.name = f"StyleGAN-{self.outclass}"
+        self.has_latent_residual = True
+        self._random_init = random_init
+        self.load_model()
+        self.set_noise_seed(0)
+        self._stop_points = self._make_stop_points()
+
+    def _mapping_net(self):
+        return self.model.g_mapping
+
+    def load_model(self):
+        checkpoint, seed = _checkpoint_or_seed("StyleGAN", f"stylegan/stylegan_{self.outclass}_{self.resolution}.pt",
+                                               self._random_init)
+        if seed is None:
+            self.model = stylegan.StyleGAN_G(self.resolution)
+            self.model.load_state_dict(torch.load(checkpoint, map_location="cpu"))
+            self.model = self.model.to(self.device)
+        else:
+            # the reference's default init, bit-for-bit (parameters created on the host under one manual seed)
+            torch.manual_seed(int(seed))
+            self.model = stylegan.StyleGAN_G(self.resolution).to(self.device)
+
+    def get_max_latents(self):
+        return 18
+
+    # ---- the fused synthesis chain ------------------------------------------------------------------------
+    def _make_stop_points(self):
+        """module name -> (chain layer, stop) for every module whose output the chain can stop at.  Block i is chain layers
+        2i (4x4: const + bias -> epi1; else conv0_up -> epi1) and 2i + 1 (conv / conv1 -> epi2)."""
+        pts = {}
+        blocks = list(self.model.g_synthesis.blocks.keys())
+        for i, name in enumerate(blocks):
+            pre = f"g_synthesis.blocks.{name}"
+            pts[pre] = (2 * i + 1, "epi")
+            for k, j in (("epi1", 2 * i), ("epi2", 2 * i + 1)):
+                pts[f"{pre}.{k}"] = pts[f"{pre}.{k}.style_mod"] = (j, "epi")
+                pts[f"{pre}.{k}.style_mod.lin"] = (j, "style")
+            if i == 0:
+                pts[f"{pre}.conv"] = (1, "conv")
+            else:
+                pts[f"{pre}.conv0_up"] = (2 * i, "conv")
+                pts[f"{pre}.conv1"] = (2 * i + 1, "conv")
+        pts["g_synthesis.torgb"] = pts["g_synthesis"] = (2 * len(blocks) - 1, "image")
+        return pts
+
+    def _synthesis(self):
+        """PackedSG1 of the whole synthesis network, re-packed when a parameter or a noise map changes."""
+        G = self.model.g_synthesis
+        noises = [m.noise for m in G.modules() if isinstance(m, stylegan.NoiseLayer)]
+        keys = (self._noise_generation,) + tuple((p._version, p.data_ptr()) for p in G.parameters()) + \
+            tuple((t._version, t.data_ptr()) for t in noises)
+        cached = getattr(self, "_synth_cache", None)
+        if cached is None or cached[0] != keys:
+            def epi(e):
+                return dict(noise_weight=e.top_epi.noise.weight, noise=e.top_epi.noise.noise, style_weight=e.style_mod.lin.weight,
+                            style_bias=e.style_mod.lin.bias)
+            layers = []
+            for i, (name, blk) in enumerate(G.blocks.items()):
+                res = int(name.split("x")[0])
+                if i == 0:
+                    c = blk.nf
+                    layers.append(dict(kind="const", weight=blk.const[0], bias=blk.bias, cin=c, cout=c, res_out=4, **epi(blk.epi1)))
+                    layers.append(dict(kind="same", weight=blk.conv.weight, bias=blk.conv.bias, cin=c, cout=c, res_out=4,
+                                       **epi(blk.epi2)))
+                else:
+                    # model.py:82: the fused transposed conv from 128^2 on, nearest upscale + conv below
+                    co, ci = blk.conv0_up.weight.shape[:2]
+                    layers.append(dict(kind="fused" if res >= 128 else "nearest", weight=blk.conv0_up.weight, bias=blk.conv0_up.bias,
+                                       cin=ci, cout=co, res_out=res, **epi(blk.epi1)))
+                    layers.append(dict(kind="same", weight=blk.conv1.weight, bias=blk.conv1.bias, cin=co, cout=co, res_out=res,
+                                       **epi(blk.epi2)))
+            packed = _native.PackedSG1(layers, G.torgb.weight[:, :, 0, 0], G.torgb.bias, G.dlatent_size)
+            self._synth_cache = cached = (keys, packed)
+        return cached[1]
+
+    def _latents(self, x):
+        """[Lw, n, 512] per-layer W latents (Lw = 1: one latent for every layer) from one latent or a list of 18
+        (wrappers.py:378-385, model.py:376-385); in Z space through the g_mapping module, so its hooks fire and edit."""
+        if isinstance(x, list):
+            assert len(x) == 18, "Must provide 1 or 18 latents"
+            ws = x if self.w_primary else [self.model.g_mapping(l) for l in x]
+            return torch.stack([w.reshape(-1, 512) for w in ws], dim=0)
+        w = x if self.w_primary else self.model.g_mapping(x)
+        return w.reshape(1, -1, 512)
+
+    def _run(self, w_layers, point):
+        j, stop = point
+        syn = self._synthesis()
+        n = w_layers.shape[1]
+        out = syn.forward(w_layers, j + 1, stop)
+        if stop == "style":
+            return out
+        res, co = syn.shapes[j]
+        if stop == "image":
+            return out.view(n, 3, res, res)
+        return out.view(n, res, res, co).permute(0, 3, 1, 2)                 # NCHW view of NHWC storage
+
+    def _fire_hooks(self, w_layers, modules):
+        """Hand every hooked module of ``modules`` (name, module) its output, each from its own run of the chain."""
+        for name, m in modules:
+            if not (len(m._forward_hooks) or len(m._forward_pre_hooks)):
+                continue
+            point = self._stop_points.get(name)
+            if point is None:
+                raise NotImplementedError(f"StyleGAN: a hook on '{name}' is not supported: the fused synthesis chain has no stop "
+                                          "point there (supported: blocks, epi1/epi2, style_mod(.lin), conv/conv0_up/conv1, "
+                                          "torgb, g_synthesis)")
+            act = self._run(w_layers, point)
+            if m(_result=act) is not act:
+                raise NotImplementedError(f"an edit on '{name}' cannot be propagated through the fused synthesis chain")
+
+    def _block_modules(self, upto):
+        for i, (name, blk) in enumerate(self.model.g_synthesis.blocks.items()):
+            if i > upto:
+                break
+            pre = f"g_synthesis.blocks.{name}"
+            for n, m in blk.named_modules(remove_duplicate=False):
+                yield (f"{pre}.{n}" if n else pre), m
+
+    def forward(self, x):
+        """wrappers.py:368-370: 0.5 * (torgb(G_synthesis(w)) + 1) for one latent or a list of 18.  Hooked stop points of the
+        synthesis network receive their activations."""
+        w_layers = self._latents(x)
+        n_blocks = len(self.model.g_synthesis.blocks)
+        G = self.model.g_synthesis
+        self._fire_hooks(w_layers, list(self._block_modules(n_blocks - 1)) + [("g_synthesis.torgb", G.torgb), ("g_synthesis", G)])
+        out = self._run(w_layers, self._stop_points["g_synthesis"])
+        return 0.5 * (out + 1)
+
+    def feature_layout(self, layer_name):
+        """Native (device) feature order of ``activations_into``: ('nhwc', (H, W, C)) for block / epilogue / conv outputs."""
+        point = self._stop_points.get(layer_name)
+        if point is None or point[1] not in ("epi", "conv"):
+            return None
+        res, co = self._synthesis().shapes[point[0]]
+        return ("nhwc", (res, res, co))
+
+    def activations_into(self, x, layer_name, out):
+        """Activations of ``layer_name`` for latents x [n, 512] (in the current primary space) as fp32 NHWC rows written into
+        ``out`` [n, H*W*C] (may be row-strided): the decomposition driver's producer for synthesis layers."""
+        j, stop = self._stop_points[layer_name]
+        w = x if self.w_primary else self.model.g_mapping(x)
+        return self._synthesis().forward(w.reshape(1, -1, 512), j + 1, stop, out=out)
+
+    def partial_forward(self, x, layer_name):
+        """wrappers.py:373-417: map Z to W through the ``g_mapping`` module (its hooks fire), stop there for any ``g_mapping*``
+        layer; otherwise run the synthesis blocks up to the first one with a child whose name contains ``layer_name`` (a
+        substring match, as the reference), firing the hooks of that block and the ones before it.  No block -> the
+        reference's RuntimeError."""
+        w_layers = self._latents(x)
+        if "g_mapping" in layer_name or layer_name == "truncation":
+            return
+        for i, (name, block) in enumerate(self.model.g_synthesis.blocks.items()):
+            prefix = f"g_synthesis.blocks.{name}"
+            leaves = [f"{prefix}.{n}" if n else prefix for n, m in block.named_modules(remove_duplicate=False) if not m._modules]
+            if any(layer_name in c for c in leaves):
+                self._fire_hooks(w_layers, list(self._block_modules(i)))
+                return
+        raise RuntimeError(f"Layer {layer_name} not encountered in partial_forward")
+
+    def set_noise_seed(self, seed):
+        """wrappers.py:420-436: every NoiseLayer gets randn(1, 1, H, W) drawn right after torch.random.manual_seed(seed)
+        (so maps of one resolution are equal), in the reference's visiting order; drawn on the host."""
+        def visit(m, name):
+            for child_name, child in m._modules.items():
+                if child is not None:
+                    visit(child, f"{name}.{child_name}")
+            if isinstance(m, stylegan.NoiseLayer):
+                H, W = [int(v) for v in name.split(".")[2].split("x")]
+                torch.random.manual_seed(seed)
+                m.noise = torch.randn(1, 1, H, W, dtype=torch.float32).to(self.device)
+        visit(self.model.g_synthesis, "g_synthesis")
+        # (new maps may reuse the freed ones' addresses: the pack key counts the re-seeds)
+        self._noise_generation = getattr(self, "_noise_generation", 0) + 1
+
+
 # ---- factories (wrappers.py:651-735) ---------------------------------------------------------------
 @singledispatch
 def get_model(name, output_class, device, **kwargs):
@@ -415,7 +629,9 @@ def get_model(name, output_class, device, **kwargs):
         assert "-" in name, "Please specify BigGAN resolution, e.g. BigGAN-512"
         from .biggan import BigGAN
         model = BigGAN(device, name.split("-")[-1], class_name=output_class, random_init=kwargs.get("random_init"))
-    elif name in ("StyleGAN", "ProGAN", "DCGAN"):
+    elif name == "StyleGAN":
+        model = StyleGAN(device, class_name=output_class, random_init=kwargs.get("random_init"))
+    elif name in ("ProGAN", "DCGAN"):
         raise RuntimeError(f"{name} is outside the B200 hot path (SURVEY.md section 2: not in any BASELINE config)")
     else:
         raise RuntimeError(f"Unknown model {name}")
